@@ -2,8 +2,12 @@
 """bench.py -- images/sec of the ViT forward hot path on B200 (BASELINE.json metric), one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload vit_b16|vit_l16_map|clip_b32|siglip_b16|siglip2_l16_512]
+                    [--dump-outputs DIR]
 
-A "step" is one forward pass of the hot path over one synthetic batch.  The default workload is BASELINE.json configs[1]:
+A "step" is one forward pass of the hot path over one synthetic batch; every timed loop below runs K steps.  Inputs and weights
+come from fixed seeds, so the same arguments give the same inputs on every run, and `--dump-outputs DIR` writes what the last timed
+step of the headline loop returned (see dump_outputs) so that two builds can be compared output for output.
+The default workload is BASELINE.json configs[1]:
 ViT-B/16 @224, batch 256 per GPU, fp16 tensor-core operands (fp32 accumulate / residual / LN / softmax), random-init weights.
   value  : whole-job images/sec with the inputs already resident in HBM (CUDA events, barrier + synchronize both sides,
            max over ranks).  Weak scaling: every rank runs its own 256-image batch; no data-path collective for ViT.
@@ -14,8 +18,8 @@ ViT-B/16 @224, batch 256 per GPU, fp16 tensor-core operands (fp32 accumulate / r
   roofline: the dominant kernel (tcgen05 GEMM) timed live with CUDA events around every launch of the timed steps.
   cpu_baseline: the CPU oracle (torch fp32, jimm semantics -- the stand-in for the reference's JAX-CPU path, which cannot
            be installed here) on a bounded sample, rank 0 / N=1 only.
-  extra_workloads (N=1): north_star's second headline (SigLIP-B/16 @256) and BASELINE configs[2] (ViT-L/16 @384 MAP, bf16), a few steps
-           each: value, e2e and the live GEMM roofline, so that they are driver-measured too.
+  extra_workloads (N=1): north_star's second headline (SigLIP-B/16 @256) and BASELINE configs[2] (ViT-L/16 @384 MAP, bf16), K steps
+           each: value, e2e and the live GEMM roofline, so that one run measures them too.
   collective (N>1): after the ViT leg every rank runs the dual-tower path the batch-sharded reference resolves with an all-gather
            (models/clip.py:183-187 under P("batch") inputs, examples/clip_inference.py:41-44): CLIP-B/32 at N<=4 (BASELINE configs[3] at N=4),
            SigLIP2-L/16 @512 at N=8 (configs[4]).  Reports pairs/s (device and e2e), the fused normalise + NVLink peer-store + logits kernel
@@ -264,6 +268,29 @@ def run_reference(args):
     return 0
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict, rank: int, world: int) -> list:
+    """Write each {name: tensor} as `directory/<name>.npy` (`<name>.rank<r>.npy` when world > 1) in float32.  The files of all ranks
+    stay within DUMP_BYTES: an array over its share is replaced by a fixed sample of its flattened elements (the same indices on
+    every run, in ascending order), so that dumps of two builds still line up element for element."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    budget = DUMP_BYTES // (world * len(arrays))
+    written = []
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > budget:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, budget // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        path = os.path.join(directory, f"{name}.npy" if world == 1 else f"{name}.rank{rank}.npy")
+        np.save(path, a)
+        written.append(path)
+    return written
+
+
 def gemm_roofline(lib, native, step_dev, steps, ms_step):
     """The dominant kernel (tcgen05 GEMM) timed live: CUDA events on the launch stream around every launch of `steps` steps."""
     from jimm_b200 import _lib
@@ -404,7 +431,7 @@ def collective_leg(args, rank, world, local, lib):
     import torch.distributed as dist
 
     wl = os.environ.get("JIMM_BENCH_COLLECTIVE_WL") or ("siglip2_l16_512" if world >= 8 else "clip_b32")  # (override: dry-run the c5 leg on fewer GPUs)
-    steps = max(2, min(args.steps, 3 if wl == "siglip2_l16_512" else 10))
+    steps = args.steps
     bw = Bench(wl, 0, rank, world, local, lib)
     m, B = bw.model, bw.B
     m.set_comm("peer")
@@ -530,11 +557,12 @@ def run_ours(args):
     e2e = bw.e2e(args.steps)
     peak_tf = roofline["peak"]
 
-    # ---- N = 1 extras: the other headline workloads, a few steps each ----
+    # ---- N = 1 extras: the other headline workloads, K steps each ----
     extras = None
     if world == 1 and not args.no_extras and args.workload == "vit_b16":
         extras = {}
-        for wl, steps in (("siglip_b16", 8), ("vit_l16_map", 5)):
+        steps = args.steps
+        for wl in ("siglip_b16", "vit_l16_map"):
             bw = None  # free the previous model's workspace before the next one is built
             torch.cuda.empty_cache()
             try:
@@ -575,6 +603,12 @@ def run_ours(args):
         cpu = {"value": ips, "unit": "images/sec", "cores": cpu_threads(), "host_cores": os.cpu_count() or 1, "kind": "port",
                "sample": f"{cb} images/step x {csteps} steps, oracle/jimm_oracle.py torch-CPU fp32 (jimm semantics)"}
 
+    if args.dump_outputs:
+        # what a caller of the headline loop receives from its last timed step: logits, or the pooled features of a bare tower
+        name = "features" if args.workload == "vit_l16_map" else "logits"
+        for path in dump_outputs(args.dump_outputs, {name: out}, rank, world):
+            print(f"bench: wrote {path}", file=sys.stderr, flush=True)
+
     if rank == 0:
         gflop = GFLOP_PER_IMG[args.workload]
         desc, _, dtype_name = WORKLOADS[args.workload]
@@ -613,7 +647,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="N=1: skip the SigLIP-B/16@256 and ViT-L/16@384 legs")
     ap.add_argument("--no-collective", action="store_true", help="N>1: skip the dual-tower leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)
