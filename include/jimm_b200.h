@@ -151,11 +151,25 @@ JIMM_API int jimm_comm_gathered(jimm_model_t* m, float** gathered, int* row_stri
 
 /* -- per-kernel entry points (device pointers; used by tests/ and the ncu harness so every kernel is individually
  *    parity- and profile-testable; SURVEY.md 8b) ------------------------------------------------------------------- */
+/* Type codes of the per-kernel entries: dtype / io_type / in_type are JIMM_F32 | JIMM_F16 | JIMM_BF16 (JIMM_F32 operands of the GEMM are
+ * read as tf32).  An out_type may also be 3 (the value of JIMM_I32), which here means "fp32 rounded to tf32": fp32 storage with the low 13
+ * mantissa bits zero, the operand format the fp32 compute mode stores between layers.  Any other out_type is rejected (JIMM_EINVAL). */
 /* C[M,N] = epi(A[M,K] . B[N,K]^T): impl 0 = tcgen05/TMA kernel, 1 = SIMT cross-check.
- * act: 0 none | 1 gelu_tanh | 2 quick_gelu; epi_mode 0 staged | 1 direct; rows_in>0 remaps output rows. */
+ * act: 0 none | 1 gelu_tanh | 2 quick_gelu; epi_mode 0 staged | 1 direct | 2 TMA store / reduce-add (0 when not applicable);
+ * rows_in>0 remaps output rows. */
 JIMM_API int jimm_k_gemm(int impl, int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, int act,
                 const float* rowadd, const float* residual, int ldr, void* out, int out_type, int ldo, int rows_in, int rows_out,
                 int row_off, int epi_mode, void* stream);
+/* The tcgen05 GEMM of jimm_k_gemm with the plan-time and run-time knobs of the model forward:
+ *   - the plan is built for M rows and run on run_M rows (0 = M; 1 <= run_M <= M): the schedule (single CTA or CTA pair, tail split)
+ *     follows run_M.  With the TMA epilogue (epi_mode 2) rows [run_M, min(M, ceil32(run_M))) are written too (see gemm_plan_run);
+ *   - reverse = 1 walks the tiles from the end (same results, bit for bit);
+ *   - tok_pad > 0: token-scatter reduce-add of the patch embedding.  A row b * tok_pad + p is added to out[b, p + tok_off, :] of an fp32
+ *     [M / tok_pad, tok_S, N] tensor (row stride ldo); rows with p + tok_off >= tok_S are dropped.  Needs residual == out, ldr == ldo,
+ *     out_type JIMM_F32, epi_mode 2, tok_pad a multiple of 32 dividing M, no rowadd / row remap. */
+JIMM_API int jimm_k_gemm_ex(int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, int act,
+                            const float* rowadd, const float* residual, int ldr, void* out, int out_type, int ldo, int rows_in, int rows_out,
+                            int row_off, int tok_pad, int tok_off, int tok_S, int run_M, int reverse, int epi_mode, void* stream);
 /* x[M,N] += A . B^T + bias through the fp32 reduce-add epilogue (CTA-pair mode, M >= 512), then -- fused -- ln_out = LayerNorm(x) row by row
  * as the last column tile of each 32-row group completes (the out-proj / FC2 + following norm of common/transformer.py:130-131).
  * counters: device int32 [M/32 + 1], zero on entry (left zero on exit).  ln_out_type JIMM_F32 stores tf32-rounded fp32. */
@@ -164,7 +178,12 @@ JIMM_API int jimm_k_gemm_residual_ln(int dtype, const void* A, int lda, const vo
                             void* stream);
 JIMM_API int jimm_k_layernorm(const float* x, int ldx, int group, int row_off, const int32_t* row_index, const float* scale, const float* bias,
                      float eps, void* out, int out_type, int ldy, int rows, int D, void* stream);
+/* reverse = 1: the same LayerNorm / attention with rows (resp. (sample, head) items) walked from the end, as every other launch of an
+ * encoder block does; the results are bit-identical to reverse = 0. */
+JIMM_API int jimm_k_layernorm_ex(const float* x, int ldx, int group, int row_off, const int32_t* row_index, const float* scale, const float* bias,
+                                 float eps, void* out, int out_type, int ldy, int rows, int D, int reverse, void* stream);
 JIMM_API int jimm_k_attention(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, void* stream);
+JIMM_API int jimm_k_attention_ex(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, int reverse, void* stream);
 JIMM_API int jimm_k_map_attention(const float* q, const void* kv, int io_type, void* out, int out_type, int B, int S, int H, void* stream);
 JIMM_API int jimm_k_patchify(const void* img, int in_type, int B, int H, int W, int C, int P, void* out, int out_type, void* stream);
 /* y = act(x) elementwise on device fp32 (act: 1 tanh-GELU == nnx.gelu, 2 QuickGELU == common/transformer.py:12-19). */

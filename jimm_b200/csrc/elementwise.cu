@@ -95,6 +95,7 @@ int layernorm_run(const float* x, int ldx, int group, int row_off, const int* ro
     set_last_error("layernorm: D=%d must be a multiple of 4 and <= 2048 (ldx=%d ldy=%d)", D, ldx, ldy);
     return -1;
   }
+  if (out_type < DT_F32 || out_type > DT_TF32) { set_last_error("layernorm: bad out_type %d", out_type); return -1; }
   if (rows <= 0) return 0;
   if (out_type == DT_F32) return ln_launch<float>(x, ldx, group, row_off, row_index, scale, bias, eps, out, ldy, rows, D, stream, reverse);
   if (out_type == DT_TF32) return ln_launch<tf32_t>(x, ldx, group, row_off, row_index, scale, bias, eps, out, ldy, rows, D, stream, reverse);
@@ -206,6 +207,7 @@ static int patchify_generic_dispatch(const void* img, int B, int H, int W, int C
 // ldk: row stride of `out` in elements (0 = P*P*C).  The vectorised kernel needs P*C and W*C to be multiples of 4 and an unpadded row.
 int patchify_run(const void* img, int in_type, int B, int H, int W, int C, int P, void* out, int out_type, cudaStream_t stream, int rows_per_sample,
                  int ldk) {
+  if (out_type < DT_F32 || out_type > DT_TF32) { set_last_error("patchify: bad out_type %d", out_type); return -1; }
   if (B <= 0) return 0;
   const int PPC = P * P * C;
   if (ldk <= 0) ldk = PPC;

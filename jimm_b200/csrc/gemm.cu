@@ -860,6 +860,7 @@ int device_sm_count() {  // of the CURRENT device (cached per device: a process 
 static int check_epi(const GemmEpilogue& e, int N) {
   if (e.out == nullptr) { set_last_error("gemm: null output"); return -1; }
   if (e.ldo < N) { set_last_error("gemm: ldo (%d) < N (%d)", e.ldo, N); return -1; }
+  if (e.out_type < DT_F32 || e.out_type > DT_TF32) { set_last_error("gemm: bad out_type %d", e.out_type); return -1; }
   return 0;
 }
 // vector accesses need aligned rows; otherwise the generic epilogue takes its scalar path (tiny head GEMMs, N = 10 classes)

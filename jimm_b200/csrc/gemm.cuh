@@ -63,7 +63,10 @@ struct GemmPlan {
 // Returns 0 or a negative status (message in jimm_last_error()).
 int gemm_plan_init(GemmPlan* plan, int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K,
                    const GemmEpilogue& epi);
-// Enqueue on `stream`; M may be overridden (<= planned M) to run on fewer rows of the same buffers.
+// Enqueue on `stream`; M may be overridden (<= planned M) to run on fewer rows of the same buffers.  The schedule (single CTA or
+// CTA pair, tail split) is chosen for the overriding M.  The TMA epilogue (mode 2) stores or reduce-adds whole 32-row boxes, clipped
+// only at the PLANNED M (the output tensor map): rows [M_override, min(planned M, ceil32(M_override))) are written too, with the
+// epilogue applied to the A rows there (whatever the buffer holds).  The LSU epilogues (modes 0 / 1) write rows < M_override only.
 int gemm_plan_run(const GemmPlan* plan, int M_override, cudaStream_t stream, int reverse = 0);
 
 // Simple SIMT reference GEMM (debug / bring-up cross-check on the GPU; never on the product path

@@ -1457,14 +1457,32 @@ int jimm_profile_end(jimm_model_t* m, double* gemm_ms, double* gemm_flops, long 
 int jimm_k_gemm(int impl, int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, int act,
                 const float* rowadd, const float* residual, int ldr, void* out, int out_type, int ldo, int rows_in, int rows_out,
                 int row_off, int epi_mode, void* stream) {
+  if (impl == 1) {
+    GemmEpilogue e;
+    e.bias = bias; e.act = act; e.rowadd = rowadd; e.residual = residual; e.ldr = ldr; e.out = out; e.out_type = out_type; e.ldo = ldo;
+    e.rows_in = rows_in; e.rows_out = rows_out; e.row_off = row_off; e.mode = epi_mode;
+    return gemm_simt_run(dtype, A, lda, B, ldb, M, N, K, e, static_cast<cudaStream_t>(stream));
+  }
+  return jimm_k_gemm_ex(dtype, A, lda, B, ldb, M, N, K, bias, act, rowadd, residual, ldr, out, out_type, ldo, rows_in, rows_out, row_off, 0, 0, 0, 0, 0,
+                        epi_mode, stream);
+}
+int jimm_k_gemm_ex(int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, int act,
+                   const float* rowadd, const float* residual, int ldr, void* out, int out_type, int ldo, int rows_in, int rows_out,
+                   int row_off, int tok_pad, int tok_off, int tok_S, int run_M, int reverse, int epi_mode, void* stream) {
+  if (run_M < 0 || run_M > M) { set_last_error("jimm_k_gemm_ex: run_M %d outside [0, M = %d]", run_M, M); return JIMM_EINVAL; }
+  if (tok_pad < 0 || (tok_pad > 0 && (residual != out || ldr != ldo || out_type != JIMM_F32 || epi_mode != 2 || rowadd || rows_in != 0 ||
+                                      tok_off < 0 || tok_S <= 0))) {
+    set_last_error("jimm_k_gemm_ex: token scatter needs residual == out, ldr == ldo, fp32 output, epi_mode 2, no row remap, tok_S > 0");
+    return JIMM_EINVAL;
+  }
   GemmEpilogue e;
   e.bias = bias; e.act = act; e.rowadd = rowadd; e.residual = residual; e.ldr = ldr; e.out = out; e.out_type = out_type; e.ldo = ldo;
   e.rows_in = rows_in; e.rows_out = rows_out; e.row_off = row_off; e.mode = epi_mode;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (impl == 1) return gemm_simt_run(dtype, A, lda, B, ldb, M, N, K, e, s);
+  e.tok_pad = tok_pad; e.tok_off = tok_off; e.tok_S = tok_S;
   GemmPlan p;
   JIMM_TRY(gemm_plan_init(&p, dtype, A, lda, B, ldb, M, N, K, e));
-  return gemm_plan_run(&p, M, s);
+  if (tok_pad > 0 && p.epi.mode != 2) { set_last_error("jimm_k_gemm_ex: token-scatter epilogue unavailable (alignment)"); return JIMM_EINVAL; }
+  return gemm_plan_run(&p, run_M > 0 ? run_M : M, static_cast<cudaStream_t>(stream), reverse != 0);
 }
 int jimm_k_gemm_residual_ln(int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, float* x, int ldx,
                             const float* ln_scale, const float* ln_bias, float eps, void* ln_out, int ln_out_type, int ln_ldo, int* counters,
@@ -1480,10 +1498,17 @@ int jimm_k_gemm_residual_ln(int dtype, const void* A, int lda, const void* B, in
 }
 int jimm_k_layernorm(const float* x, int ldx, int group, int row_off, const int32_t* row_index, const float* scale, const float* bias,
                      float eps, void* out, int out_type, int ldy, int rows, int D, void* stream) {
-  return layernorm_run(x, ldx, group, row_off, row_index, scale, bias, eps, out, out_type, ldy, rows, D, static_cast<cudaStream_t>(stream));
+  return jimm_k_layernorm_ex(x, ldx, group, row_off, row_index, scale, bias, eps, out, out_type, ldy, rows, D, 0, stream);
+}
+int jimm_k_layernorm_ex(const float* x, int ldx, int group, int row_off, const int32_t* row_index, const float* scale, const float* bias,
+                        float eps, void* out, int out_type, int ldy, int rows, int D, int reverse, void* stream) {
+  return layernorm_run(x, ldx, group, row_off, row_index, scale, bias, eps, out, out_type, ldy, rows, D, static_cast<cudaStream_t>(stream), reverse != 0);
 }
 int jimm_k_attention(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, void* stream) {
-  return attention_run(qkv, io_type, out, out_type, B, S, H, causal, static_cast<cudaStream_t>(stream));
+  return jimm_k_attention_ex(qkv, io_type, out, out_type, B, S, H, causal, 0, stream);
+}
+int jimm_k_attention_ex(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, int reverse, void* stream) {
+  return attention_run(qkv, io_type, out, out_type, B, S, H, causal, static_cast<cudaStream_t>(stream), reverse != 0);
 }
 int jimm_k_map_attention(const float* q, const void* kv, int io_type, void* out, int out_type, int B, int S, int H, void* stream) {
   return map_attention_run(q, kv, io_type, out, out_type, B, S, H, static_cast<cudaStream_t>(stream));

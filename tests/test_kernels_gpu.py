@@ -315,13 +315,22 @@ def test_bad_arguments_return_errors(lib):
     A7 = torch.zeros(8, 7, device=DEV).half()
     rc = lib.jimm_k_gemm(0, F16, ptr(A7), 7, ptr(A7), 7, 8, 8, 7, None, 0, None, None, 0, ptr(out), F32, 8, 0, 0, 0, 0, stream())
     assert rc == -1 and b"16-byte aligned" in lib.jimm_last_error()
+    for bad in (-1, 4, 7):  # out_type codes are 0..3 (3 = fp32 rounded to tf32)
+        rc = lib.jimm_k_gemm(0, F16, ptr(A), 8, ptr(A), 8, 8, 8, 8, None, 0, None, None, 0, ptr(out), bad, 8, 0, 0, 0, 0, stream())
+        assert rc == -1 and b"out_type" in lib.jimm_last_error()
+        rc = lib.jimm_k_gemm(1, F16, ptr(A), 8, ptr(A), 8, 8, 8, 8, None, 0, None, None, 0, ptr(out), bad, 8, 0, 0, 0, 0, stream())
+        assert rc == -1 and b"out_type" in lib.jimm_last_error()
+        y = torch.zeros(2, 8, device=DEV)
+        rc = lib.jimm_k_layernorm(ptr(y), 8, 1, 0, None, ptr(y), ptr(y), 1e-6, ptr(y), bad, 8, 2, 8, stream())
+        assert rc == -1 and b"out_type" in lib.jimm_last_error()
     x = torch.zeros(2, 6, device=DEV)
     rc = lib.jimm_k_layernorm(ptr(x), 6, 1, 0, None, ptr(x), ptr(x), 1e-6, ptr(x), F32, 6, 2, 6, stream())
     assert rc == -1
 
 
 @pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16, torch.float32])
-@pytest.mark.parametrize("M,N,K", [(1000, 768, 256), (50432 // 8, 768, 768), (2000, 512, 2048), (777, 1152, 320), (5000, 1024, 512)])
+@pytest.mark.parametrize("M,N,K", [(1000, 768, 256), (50432 // 8, 768, 768), (2000, 512, 2048), (777, 1152, 320), (5000, 1024, 512),
+                                   (1024, 128, 256), (1536, 256, 256), (1000, 384, 512), (2048, 1280, 320), (1024, 1536, 256), (600, 2048, 256)])
 def test_gemm_residual_with_fused_layernorm(lib, dtype, M, N, K):
     """x += A B^T + bias, then LayerNorm(x) written by the warp that completes each 32-row group (also in place over the A operand, as the
     out-projection does): x bit-identical to the unfused kernel, the normalised rows equal to the LayerNorm kernel on that x."""
