@@ -170,12 +170,6 @@ JIMM_API int jimm_k_gemm(int impl, int dtype, const void* A, int lda, const void
 JIMM_API int jimm_k_gemm_ex(int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, int act,
                             const float* rowadd, const float* residual, int ldr, void* out, int out_type, int ldo, int rows_in, int rows_out,
                             int row_off, int tok_pad, int tok_off, int tok_S, int run_M, int reverse, int epi_mode, void* stream);
-/* x[M,N] += A . B^T + bias through the fp32 reduce-add epilogue (CTA-pair mode, M >= 512), then -- fused -- ln_out = LayerNorm(x) row by row
- * as the last column tile of each 32-row group completes (the out-proj / FC2 + following norm of common/transformer.py:130-131).
- * counters: device int32 [M/32 + 1], zero on entry (left zero on exit).  ln_out_type JIMM_F32 stores tf32-rounded fp32. */
-JIMM_API int jimm_k_gemm_residual_ln(int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, float* x, int ldx,
-                            const float* ln_scale, const float* ln_bias, float eps, void* ln_out, int ln_out_type, int ln_ldo, int* counters,
-                            void* stream);
 JIMM_API int jimm_k_layernorm(const float* x, int ldx, int group, int row_off, const int32_t* row_index, const float* scale, const float* bias,
                      float eps, void* out, int out_type, int ldy, int rows, int D, void* stream);
 /* reverse = 1: the same LayerNorm / attention with rows (resp. (sample, head) items) walked from the end, as every other launch of an

@@ -80,7 +80,6 @@ SIGNATURES = {
     "jimm_profile_end": (_i, [_vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_longlong)]),
     "jimm_k_gemm": (_i, [_i, _i, _vp, _i, _vp, _i, _i, _i, _i, _fp, _i, _fp, _fp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "jimm_k_gemm_ex": (_i, [_i, _vp, _i, _vp, _i, _i, _i, _i, _fp, _i, _fp, _fp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
-    "jimm_k_gemm_residual_ln": (_i, [_i, _vp, _i, _vp, _i, _i, _i, _i, _fp, _fp, _i, _fp, _fp, _f, _vp, _i, _i, _ip, _vp]),
     "jimm_k_layernorm": (_i, [_fp, _i, _i, _i, _ip, _fp, _fp, _f, _vp, _i, _i, _i, _i, _vp]),
     "jimm_k_layernorm_ex": (_i, [_fp, _i, _i, _i, _ip, _fp, _fp, _f, _vp, _i, _i, _i, _i, _i, _vp]),
     "jimm_k_attention": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp]),

@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "_build")
 LIB = os.path.join(HERE, "libjimm_b200.so")
-SOURCES = ["gemm.cu", "attention.cu", "attention_tc.cu", "attention_tc_split.cu", "attention_tc_long.cu", "elementwise.cu", "pack.cu", "comm.cu", "preprocess.cu", "postprocess.cu", "probe.cu", "model.cu"]
+SOURCES = ["gemm.cu", "attention.cu", "attention_tc.cu", "attention_tc_long.cu", "elementwise.cu", "pack.cu", "comm.cu", "preprocess.cu", "postprocess.cu", "probe.cu", "model.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -276,11 +276,7 @@ static int attn_launch(const void* qkv, void* out, int B, int S, int H, int caus
 
 int attention_run(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, cudaStream_t stream, int reverse) {
   if (B <= 0 || S <= 0) return 0;
-  const char* env = getenv("JIMM_ATTN_IMPL");  // "flash" forces the mma.sync flash kernel, "split" the column-split tcgen05 variant (A/B comparison, bisection)
-  if (env && strcmp(env, "split") == 0) {  // the two-threads-per-row variant of the S <= 256 kernel (slower; kept for A/B runs and tests)
-    const int rc = attention_tc_split_run(qkv, io_type, out, out_type, B, S, H, causal, stream, reverse);
-    if (rc <= 0) return rc;
-  }
+  const char* env = getenv("JIMM_ATTN_IMPL");  // "flash" forces the mma.sync flash kernel for every S (bisection)
   if (!(env && strcmp(env, "flash") == 0)) {
     int rc = attention_tc_run(qkv, io_type, out, out_type, B, S, H, causal, stream, reverse);
     if (rc <= 0) return rc;

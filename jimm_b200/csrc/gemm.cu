@@ -31,8 +31,6 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include <type_traits>
-
 #include "common.cuh"
 
 namespace jimm {
@@ -79,13 +77,6 @@ struct EpiDev {
   // few of the CTA pairs.  When tail * parts <= #pairs those tiles are cut into `parts` (2 or 4) column slices of 256 / parts columns,
   // so the last round takes ~1 / parts of a round: virtual tiles [0, full) are whole tiles, [full, full + tail * parts) the slices.
   int full_tiles, tail_parts;
-  // fused LayerNorm of completed row groups (see GemmEpilogue)
-  const float* ln_scale;
-  const float* ln_bias;
-  void* ln_out;
-  int* ln_cnt;
-  int ln_out_type, ln_ldo;
-  float ln_eps;
   int vec;  // 1: N / ldo / ldr multiples of 4 and 16-byte aligned pointers -> vector accesses allowed (generic path)
 };
 
@@ -149,157 +140,6 @@ struct Traits<float> {
   static constexpr int KIND = 1, FMT = 2;
 };
 
-
-// ---- fused LayerNorm of completed 32-row groups (CTA-pair reduce-add epilogue) -----------------------------------------------------
-// Who normalises: NOT the epilogue warps.  A first version let the epilogue warp that completed a row group normalise it in place; every
-// such warp then came late to its next tile, the accumulator hand-off (all 8 warps of both CTAs) stalled the MMA issuer once per round, and
-// the step went from 10.2 to 17.5 ms.  Here the epilogue warps only PUBLISH (wait for their reduce-adds, bump the group's counter, and the
-// one that completes a group pushes its index into a shared-memory ring); the CTA's otherwise idle warps (2, 3 and, in the non-leader CTA,
-// 1) pop indices and normalise, off the MMA / epilogue critical path.  The rows are read back with ld.global.cg (they were just
-// reduce-added in L2; L1 is bypassed) in batches whose loads are all issued back to back, double-buffered in registers.
-// Same arithmetic as layernorm_kernel (elementwise.cu): fp32, var = max(0, E[x^2] - E[x]^2).  NV = D / 128 float4 per lane per row.
-static constexpr int ACT_FUSE_LN = 7;  // internal marker in the kernel's ACT slot (OUT_F32_ADD has no activation)
-static constexpr int LNQ = 240;        // ring slots; with head / tail / done it fits the (unused, for this epilogue) per-tile bias copy
-struct LnQueue {
-  int head, tail, done, pad;
-  int slot[LNQ];  // -1 = empty, else a row-group index
-};
-static_assert(sizeof(LnQueue) <= BIAS_BYTES, "LN work queue must fit the bias staging area");
-
-template <typename OutT, int NV>
-__device__ __forceinline__ void ln_rows_nv(const EpiDev& e, int row0, int lane) {
-  constexpr int R0 = 12 / NV;
-  constexpr int R = R0 < 1 ? 1 : (R0 > 8 ? 8 : R0);  // rows per batch: <= 12 float4 per lane per buffer
-  constexpr bool DOUBLE = NV <= 9;                   // wider rows: one buffer (a row's loads still go out back to back)
-  const float inv_d = 1.0f / static_cast<float>(NV * 128);
-  const float4* sc = reinterpret_cast<const float4*>(e.ln_scale);
-  const float4* bi = reinterpret_cast<const float4*>(e.ln_bias);
-  const float* xbase = static_cast<const float*>(e.out);
-  const int ldx = e.ldo, ldh = e.ln_ldo;
-  const float eps = e.ln_eps;
-  OutT* hbase = static_cast<OutT*>(e.ln_out);
-  const int rows = min(32, e.M - row0);
-  float4 a[R][NV];
-  float4 b[DOUBLE ? R : 1][DOUBLE ? NV : 1];
-#define JIMM_LN_LOAD(buf, r0_)                                                                                          \
-  _Pragma("unroll") for (int i = 0; i < R; ++i) { /* unconditional (row clamped): the buffers stay in registers */     \
-    const float4* xr = reinterpret_cast<const float4*>(xbase + static_cast<size_t>(row0 + min((r0_) + i, rows - 1)) * ldx); \
-    _Pragma("unroll") for (int j = 0; j < NV; ++j) buf[i][j] = __ldcg(xr + lane + 32 * j);                              \
-  }
-#define JIMM_LN_PROCESS(buf, r0_)                                                                                       \
-  _Pragma("unroll") for (int i = 0; i < R; ++i) {                                                                       \
-    if ((r0_) + i < rows) {                                                                                             \
-      float s = 0.f, s2 = 0.f;                                                                                          \
-      _Pragma("unroll") for (int j = 0; j < NV; ++j) {                                                                  \
-        const float4 v = buf[i][j];                                                                                     \
-        s += v.x + v.y + v.z + v.w;                                                                                     \
-        s2 += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;                                                            \
-      }                                                                                                                 \
-      s = warp_sum(s);                                                                                                  \
-      s2 = warp_sum(s2);                                                                                                \
-      const float mean = s * inv_d;                                                                                     \
-      const float rstd = rsqrtf(fmaxf(s2 * inv_d - mean * mean, 0.0f) + eps);                                           \
-      OutT* orow = hbase + static_cast<size_t>(row0 + (r0_) + i) * ldh;                                                 \
-      _Pragma("unroll") for (int j = 0; j < NV; ++j) {                                                                  \
-        const int idx = lane + 32 * j;                                                                                  \
-        const float4 v = buf[i][j], g = __ldg(sc + idx), bb = __ldg(bi + idx);                                          \
-        float4 y;                                                                                                       \
-        y.x = (v.x - mean) * rstd * g.x + bb.x;                                                                         \
-        y.y = (v.y - mean) * rstd * g.y + bb.y;                                                                         \
-        y.z = (v.z - mean) * rstd * g.z + bb.z;                                                                         \
-        y.w = (v.w - mean) * rstd * g.w + bb.w;                                                                         \
-        if constexpr (std::is_same<OutT, float>::value) {                                                               \
-          reinterpret_cast<float4*>(orow)[idx] = make_float4(round_tf32(y.x), round_tf32(y.y), round_tf32(y.z), round_tf32(y.w)); \
-        } else {                                                                                                        \
-          uint2 pk;                                                                                                     \
-          constexpr int ot = std::is_same<OutT, __half>::value ? DT_F16 : DT_BF16;                                      \
-          pk.x = pack2(y.x, y.y, ot);                                                                                   \
-          pk.y = pack2(y.z, y.w, ot);                                                                                   \
-          reinterpret_cast<uint2*>(orow)[idx] = pk;                                                                     \
-        }                                                                                                               \
-      }                                                                                                                 \
-    }                                                                                                                   \
-  }
-  if constexpr (DOUBLE) {
-    JIMM_LN_LOAD(a, 0)
-#pragma unroll 1
-    for (int r0 = 0; r0 < rows; r0 += 2 * R) {
-      JIMM_LN_LOAD(b, r0 + R)
-      JIMM_LN_PROCESS(a, r0)
-      JIMM_LN_LOAD(a, r0 + 2 * R)
-      JIMM_LN_PROCESS(b, r0 + R)
-    }
-  } else {
-#pragma unroll 1
-    for (int r0 = 0; r0 < rows; r0 += R) {
-      JIMM_LN_LOAD(a, r0)
-      JIMM_LN_PROCESS(a, r0)
-    }
-  }
-#undef JIMM_LN_LOAD
-#undef JIMM_LN_PROCESS
-}
-
-// OutT = the GEMM's operand type (the normalised rows are the next GEMM's A operand; float = tf32-rounded fp32)
-template <typename OutT>
-__device__ __forceinline__ void ln_rows_dispatch(const EpiDev& e, int row0, int lane) {
-  switch (e.N >> 7) {  // gemm_fuses_ln() admits exactly these widths
-    case 1: ln_rows_nv<OutT, 1>(e, row0, lane); break;
-    case 2: ln_rows_nv<OutT, 2>(e, row0, lane); break;
-    case 3: ln_rows_nv<OutT, 3>(e, row0, lane); break;
-    case 4: ln_rows_nv<OutT, 4>(e, row0, lane); break;
-    case 6: ln_rows_nv<OutT, 6>(e, row0, lane); break;
-    case 8: ln_rows_nv<OutT, 8>(e, row0, lane); break;
-    case 9: ln_rows_nv<OutT, 9>(e, row0, lane); break;
-    case 10: ln_rows_nv<OutT, 10>(e, row0, lane); break;
-    case 12: ln_rows_nv<OutT, 12>(e, row0, lane); break;
-    case 16: ln_rows_nv<OutT, 16>(e, row0, lane); break;
-    default: break;
-  }
-}
-
-// Epilogue side (lane 0 of an epilogue warp): this thread's reduce-adds of `cols` columns into row group `rg` have been ISSUED; wait for
-// their completion, publish, and if that completes the rows (all N columns added, by whichever CTAs handled the other column tiles) queue
-// the group for this CTA's LayerNorm warps.
-__device__ __forceinline__ void ln_publish(const EpiDev& e, LnQueue* q, int rg, int cols) {
-  tma_store_wait_all();  // the bulk reduce-adds of this thread are complete (performed in L2) ...
-  __threadfence();       // ... and ordered before the counter update (release; cumulative over what this thread observed)
-  const int old = atomicAdd(e.ln_cnt + rg, cols);
-  if (old + cols == e.N) {
-    e.ln_cnt[rg] = 0;  // self-cleaning for the next launch
-    __threadfence();   // acquire side: the other contributors' adds are ordered before the consumer's loads
-    const int t = atomicAdd(&q->tail, 1);
-    volatile int* s = &q->slot[t % LNQ];
-    while (*s != -1) __nanosleep(64);  // ring full: the consumers always make progress
-    *s = rg;
-  }
-}
-
-// LayerNorm warp: pop row groups until every epilogue warp of this CTA has finished publishing and the ring is drained.
-template <typename OutT>
-__device__ __forceinline__ void ln_worker(const EpiDev& e, LnQueue* q, int lane) {
-  for (;;) {
-    int rg = -2;
-    if (lane == 0) {
-      const int t = atomicAdd(&q->head, 1);
-      volatile int* s = &q->slot[t % LNQ];
-      for (;;) {
-        if (*s >= 0) {
-          const int v = atomicExch(&q->slot[t % LNQ], -1);
-          if (v >= 0) { rg = v; break; }
-        }
-        // `done` is bumped after a warp's last push (tail already final for that warp): once all have, tickets >= tail get nothing
-        if (*reinterpret_cast<volatile int*>(&q->done) == EPI_WARPS && t >= *reinterpret_cast<volatile int*>(&q->tail)) break;
-        __nanosleep(256);
-      }
-      __threadfence();
-    }
-    rg = __shfl_sync(0xffffffffu, rg, 0);
-    if (rg < 0) return;
-    ln_rows_dispatch<OutT>(e, rg * 32, lane);
-  }
-}
-
 // ---- TMA epilogue for one 128 x 128 half-tile owned by one epilogue warp's lane quarter (thread = row) ------------
 // 16-bit outputs: 64 columns per 32 x 128 B box (two x32 TMEM loads); 32-bit outputs: 32 columns per box.
 // `release()` hands the accumulator back to the MMA issuer; it is called as soon as this warp's LAST tcgen05.ld has completed, i.e.
@@ -327,7 +167,7 @@ __device__ __forceinline__ void epilogue_tma(const CUtensorMap* map_c, const Epi
       float4 b4;
       if constexpr (OUT == OUT_F32_ADD) {
         // straight from global (warp-uniform address, L1 broadcast): the residual epilogue has no per-tile bias staging and therefore no
-        // CTA-wide barrier -- its warps run independently, one of them may be normalising a finished row group (ln_signal)
+        // CTA-wide barrier -- its warps run independently
         b4 = (sbias != nullptr && n_tile0 + c + j < N) ? __ldg(reinterpret_cast<const float4*>(sbias + n_tile0 + c + j)) : make_float4(0.f, 0.f, 0.f, 0.f);
       } else {
         b4 = *reinterpret_cast<const float4*>(sbias + c + j);
@@ -502,8 +342,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
   constexpr int NSTAGE = PAIR ? P_STAGES : STAGES;
   constexpr int B_BYTES = PAIR ? P_B_STAGE_BYTES : B_STAGE_BYTES;
   constexpr int TILE_M = PAIR ? 2 * BM : BM;
-  constexpr bool FUSE_LN = PAIR && OUT == OUT_F32_ADD && ACT == ACT_FUSE_LN;  // see "fused LayerNorm" above
-  constexpr int EPI_ACT = ACT == ACT_FUSE_LN ? static_cast<int>(ACT_NONE) : ACT;
 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -513,7 +351,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
   constexpr int EPI_BUFS = PAIR ? P_EPI_BUFS : 1;
   constexpr int EPI_REGION = EPI_BUFS * EPI_STAGE_BYTES;
   float* sbias = reinterpret_cast<float*>(epi_stage + EPI_REGION);
-  LnQueue* lnq = reinterpret_cast<LnQueue*>(sbias);  // FUSE_LN only: the reduce-add epilogue reads its bias from global memory
   uint64_t* bars = reinterpret_cast<uint64_t*>(epi_stage + EPI_REGION + BIAS_BYTES);
   uint64_t* full_bar = bars;                    // [NSTAGE]
   uint64_t* empty_bar = bars + NSTAGE;          // [NSTAGE]
@@ -553,12 +390,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
   if (warp_idx == 2) {
     if constexpr (PAIR) tmem_alloc_pair(tmem_ptr_smem, TMEM_COLS);
     else tmem_alloc(tmem_ptr_smem, TMEM_COLS);
-  }
-  if constexpr (FUSE_LN) {
-    if (warp_idx == 3) {
-      for (int i = lane; i < LNQ; i += 32) lnq->slot[i] = -1;
-      if (lane == 0) lnq->head = lnq->tail = lnq->done = 0;
-    }
   }
   tcgen05_fence_before();
   if constexpr (PAIR) cluster_sync_all();  // the peer's barriers must be initialised before any remote arrive / multicast commit
@@ -639,18 +470,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         }
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
       }
-    } else if constexpr (FUSE_LN) {
-      ln_worker<T>(epi, lnq, lane);  // the non-leader CTA issues no MMAs: its warp 1 normalises too
     }
-  } else if (warp_idx < 4) {
-    if constexpr (FUSE_LN) ln_worker<T>(epi, lnq, lane);
-  } else {
+  } else if (warp_idx >= 4) {
     // ===================== epilogue =====================
     const int q = warp_idx & 3;            // the TMEM lane quarter this warp may access (hardware rule: warp % 4)
     const int half = (warp_idx - 4) >> 2;  // column half of the 256-wide accumulator this warp drains
     int acc = 0;
     uint32_t acc_phase = 0, box_count = 0;
-    int ln_rg = -1, ln_cols = 0;  // row group / column count of this warp's previous tile, not yet published (fused LayerNorm)
     const uint32_t tmem_empty_leader0 = PAIR ? mapa_shared(smem_u32(&tmem_empty_bar[0]), 0) : 0u;
     for (int tile = tile0; tile < num_tiles; tile += tile_step) {
       const TileCoord tc = decode_tile(epi, epi.reverse ? num_tiles - 1 - tile : tile, n_tiles);
@@ -658,7 +484,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
       const int n_tile0 = tc.n_blk * BN + tc.n_off;  // first column of this (possibly sliced) tile
       const int c_len = tc.width / 2;                // accumulator columns per column half
       const int row_base = m_blk * TILE_M + static_cast<int>(cta_rank) * BM + q * 32;
-      if constexpr (OUT != OUT_GENERIC && OUT != OUT_F32_ADD) {  // (OUT_F32_ADD: bias from global; its staging area may hold the LN queue)
+      if constexpr (OUT != OUT_GENERIC && OUT != OUT_F32_ADD) {  // (OUT_F32_ADD: bias from global, so its warps need no barrier)
         // per-tile bias copy (one coalesced 128-bit load per lane of two warps), overlapped with the wait for the MMAs
         named_bar_sync(1, EPI_WARPS * 32);  // every epilogue warp is done with the previous tile's bias
         if (q == 0) {  // sbias[c] = bias[n_tile0 + c] for the accumulator columns c of this half
@@ -685,16 +511,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         release();
       } else if constexpr (OUT != OUT_GENERIC) {
         if (row_base < M) {
-          epilogue_tma<OUT, EPI_ACT, EPI_BUFS>(&map_c, epi, taddr, OUT == OUT_F32_ADD ? epi.bias : sbias, epi_stage + (warp_idx - 4) * EPI_BUFS * EPI_BUF_BYTES,
+          epilogue_tma<OUT, ACT, EPI_BUFS>(&map_c, epi, taddr, OUT == OUT_F32_ADD ? epi.bias : sbias, epi_stage + (warp_idx - 4) * EPI_BUFS * EPI_BUF_BYTES,
                                            lane, row_base, n_tile0, half * c_len, c_len, box_count, release);
-          if constexpr (FUSE_LN) {
-            // Publishing is deferred by one tile: the PREVIOUS tile's reduce-adds were issued a whole mainloop ago, so waiting for them
-            // costs nothing; this tile's accumulator has already been handed back, so the MMA issuer is not held up either.
-            if (lane == 0 && ln_rg >= 0) ln_publish(epi, lnq, ln_rg, ln_cols);
-            const int cols = min(c_len, N - (n_tile0 + half * c_len));
-            ln_rg = cols > 0 ? row_base >> 5 : -1;
-            ln_cols = cols;
-          }
         } else {
           release();
         }
@@ -704,13 +522,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         release();
       }
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-    }
-    if constexpr (FUSE_LN) {
-      if (lane == 0) {
-        if (ln_rg >= 0) ln_publish(epi, lnq, ln_rg, ln_cols);
-        __threadfence_block();
-        atomicAdd(&lnq->done, 1);
-      }
     }
     if constexpr (OUT != OUT_GENERIC) {
       if (lane == 0) tma_store_wait_all();
@@ -820,22 +631,6 @@ int make_tensor_map_3d(CUtensorMap* map, int dtype, const void* ptr, int B, int 
   if (r != CUDA_SUCCESS) { set_last_error("cuTensorMapEncodeTiled(3d) failed: CUresult %d", static_cast<int>(r)); return -3; }
   return 0;
 }
-// [B, S, N] view with a 32-row x 64-byte box (SWIZZLE_64B): the per-warp output box of the column-split attention kernel
-int make_tensor_map_3d_box64(CUtensorMap* map, int dtype, const void* ptr, int B, int S, int N, int ld) {
-  PFN_encodeTiled enc = get_encode_fn();
-  if (!enc) return -3;
-  const size_t es = dtype_size(dtype);
-  CUtensorMapDataType dt = (dtype == DT_F32 || dtype == DT_TF32) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
-                                           : (dtype == DT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
-  cuuint64_t dims[3] = {static_cast<cuuint64_t>(N), static_cast<cuuint64_t>(S), static_cast<cuuint64_t>(B)};
-  cuuint64_t strides[2] = {static_cast<cuuint64_t>(ld) * es, static_cast<cuuint64_t>(S) * ld * es};
-  cuuint32_t box[3] = {static_cast<cuuint32_t>(64 / es), 32, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(map, dt, 3, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_last_error("cuTensorMapEncodeTiled(3d, 64 B box) failed: CUresult %d", static_cast<int>(r)); return -3; }
-  return 0;
-}
 static int make_map_3d_f32(CUtensorMap* map, const void* ptr, int B, int S, int N, int ld) { return make_tensor_map_3d(map, DT_F32, ptr, B, S, N, ld); }
 
 int make_tensor_map_2d(CUtensorMap* map, int dtype, const void* ptr, int rows, int cols, int ld, int box_rows) {
@@ -910,8 +705,6 @@ static EpiDev to_dev(const GemmEpilogue& e, int M, int N) {
   d.reverse = e.reverse;
   d.full_tiles = ((M + BM - 1) / BM) * ((N + BN - 1) / BN);  // overwritten by the pair-mode launch (its row blocks are 2 * BM)
   d.tail_parts = 1;
-  d.ln_scale = e.ln_scale; d.ln_bias = e.ln_bias; d.ln_out = e.ln_out; d.ln_cnt = nullptr;  // enabled by the pair-mode launch only
-  d.ln_out_type = e.ln_out_type; d.ln_ldo = e.ln_ldo; d.ln_eps = e.ln_eps;
   d.vec = epi_vec_ok(e, N);
   static int dbg = -1;
   if (dbg < 0) { const char* env = getenv("JIMM_GEMM_DEBUG"); dbg = env ? atoi(env) : 0; }
@@ -952,7 +745,6 @@ static int launch_one(const GemmPlan* p, int M, cudaStream_t stream) {
     }
     d.full_tiles = parts > 1 ? tiles - tail : tiles;
     d.tail_parts = parts;
-    if (ACT == ACT_FUSE_LN) d.ln_cnt = p->epi.ln_cnt;
     const int vtiles = d.full_tiles + (tiles - d.full_tiles) * parts;
     const int pairs = vtiles < max_pairs ? vtiles : max_pairs;
     JIMM_CUDA_CHECK(launch_k(gemm_tcgen05_kernel<T, OUT, ACT, true>, dim3(2 * pairs), dim3(NUM_THREADS), SMEM_BYTES, stream, 2, true,
@@ -981,23 +773,13 @@ template <typename T>
 static int launch_tc(const GemmPlan* p, int M, cudaStream_t stream) {
   const GemmEpilogue& e = p->epi;
   if (e.mode != 2) return launch_one<T, OUT_GENERIC, ACT_NONE>(p, M, stream);
-  if (e.residual) return gemm_fuses_ln(p, M) ? launch_one<T, OUT_F32_ADD, ACT_FUSE_LN>(p, M, stream) : launch_one<T, OUT_F32_ADD, ACT_NONE>(p, M, stream);
+  if (e.residual) return launch_one<T, OUT_F32_ADD, ACT_NONE>(p, M, stream);
   switch (e.out_type) {
     case DT_F16: return launch_act<T, OUT_H16>(p, M, stream);
     case DT_BF16: return launch_act<T, OUT_BF16>(p, M, stream);
     case DT_TF32: return launch_act<T, OUT_TF32>(p, M, stream);
     default: return launch_act<T, OUT_F32>(p, M, stream);
   }
-}
-
-// Will gemm_plan_run(p, M) normalise the finished rows itself (GemmEpilogue::ln_*)?  Same predicate as launch_one.
-int gemm_fuses_ln(const GemmPlan* p, int M_override) {
-  const int M = (M_override > 0 && M_override <= p->M) ? M_override : p->M;
-  const int nv = p->N >> 7;
-  const bool width_ok = p->N % 128 == 0 && (nv <= 4 || nv == 6 || (nv >= 8 && nv <= 10) || nv == 12 || nv == 16);  // ln_rows_dispatch
-  // the normalised rows are written in this GEMM's operand type (they are the next GEMM's A operand)
-  const int want = p->dtype == DT_F16 ? DT_F16 : p->dtype == DT_BF16 ? DT_BF16 : DT_TF32;
-  return p->epi.ln_cnt != nullptr && p->epi.ln_out_type == want && width_ok && p->epi.mode == 2 && p->epi.residual != nullptr && p->epi.tok_pad == 0 && pair_mode_enabled() && M >= 512;
 }
 
 int gemm_plan_run(const GemmPlan* p0, int M_override, cudaStream_t stream, int reverse) {

@@ -39,17 +39,6 @@ struct GemmEpilogue {
   //    no rowadd / row remap and residual == out) -- falls back to 0 when not applicable;
   // 0: smem-staged, coalesced LSU stores; 1: direct row-per-thread LSU stores
   int mode = 2;
-  // Fused LayerNorm of the UPDATED residual rows (fp32 reduce-add epilogue in CTA-pair mode only): when the last column tile of a
-  // 32-row group has been added, the epilogue warp that completed it normalises those rows (nnx.LayerNorm fast variance,
-  // common/transformer.py:130-131: the norm that follows `x + attn(...)` / `x + mlp(...)`) and writes them as the next GEMM's A operand.
-  // ln_cnt: int32 [ceil(M/32)] completion counters, zero before the first launch (the kernel resets them).  ln_out may alias this
-  // GEMM's A operand (rows whose tiles are all done are no longer read).
-  const float* ln_scale = nullptr;
-  const float* ln_bias = nullptr;
-  void* ln_out = nullptr;
-  int ln_out_type = DT_F16, ln_ldo = 0;
-  float ln_eps = 1e-6f;
-  int* ln_cnt = nullptr;
 };
 
 struct GemmPlan {
@@ -73,9 +62,6 @@ int gemm_plan_run(const GemmPlan* plan, int M_override, cudaStream_t stream, int
 // unless JIMM_GEMM_IMPL=simt is set for bisection).
 int gemm_simt_run(int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const GemmEpilogue& epi,
                   cudaStream_t stream);
-
-// 1 when gemm_plan_run(plan, M_override) will apply the plan's fused LayerNorm (fp32 reduce-add epilogue in CTA-pair mode)
-int gemm_fuses_ln(const GemmPlan* plan, int M_override);
 
 int device_sm_count();
 

@@ -75,8 +75,6 @@ int attention_run(const void* qkv, int io_type, void* out, int out_type, int B, 
 int attention_tc_run(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, cudaStream_t stream, int reverse = 0);
 
 // tcgen05 two-pass variant for S > 256, non-causal (attention_tc_long.cu); returns 1 when not handled.
-// two-threads-per-row variant of attention_tc_run (attention_tc_split.cu; JIMM_ATTN_IMPL=split)
-int attention_tc_split_run(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, cudaStream_t stream, int reverse = 0);
 int attention_tc_long_run(const void* qkv, int io_type, void* out, int out_type, int B, int S, int H, int causal, cudaStream_t stream, int reverse = 0);
 
 // MAP-head attention with a single (input-independent) probe query (common/vit.py:96-97).

@@ -163,7 +163,6 @@ struct TextWs {
   void* big = nullptr;    // qkv | mlp hidden
   void* pooled = nullptr; // [Bmax, Dt]
   int* idx = nullptr;     // [Bmax] EOT positions
-  int* ln_cnt = nullptr;  // fused-LayerNorm completion counters, one per 32 rows
 };
 
 struct Workspace {
@@ -179,7 +178,6 @@ struct Workspace {
   float* nrm_i = nullptr; // normalised
   float* nrm_t = nullptr;
   void* in_img = nullptr; // host-path staging: image batch (fp32 worst case)
-  int* ln_cnt = nullptr;     // fused-LayerNorm completion counters (one per 32 rows of the residual stream), zero between launches
   uint8_t* in_u8 = nullptr;  // host-path staging of raw uint8 RGB frames (jimm_vit_forward_host_u8); grown on demand
   size_t in_u8_bytes = 0;
   int32_t* in_ids = nullptr;
@@ -233,10 +231,6 @@ struct jimm_model {
   int epi_mode_16 = 2;  // epilogue mode for 16-bit no-residual outputs (2 = TMA store)
   int epi_mode_res = 2; // epilogue mode for fp32 residual outputs (2 = TMA reduce-add into the residual stream)
   bool l2_alternate = true;  // JIMM_L2_ALTERNATE=0 disables the alternating walk direction
-  // JIMM_FUSE_LN=1: the out-proj / FC2 GEMMs normalise the rows they complete (gemm.cu, "fused LayerNorm").  Off by default: it removes
-  // two launches per block but is SLOWER on every measured shape (14.1 vs 11.5 ms/step, ViT-B/16 B=256) -- the row read-back competes with
-  // the GEMM's own TMA traffic for the SM<->L2 ports that already bound it (DESIGN.md section 3).  Kept for A/B runs and covered by tests.
-  bool fuse_ln = false;
   bool simt = false;    // JIMM_GEMM_IMPL=simt: bisection aid, routes every GEMM through the SIMT cross-check kernel
   // CUDA-graph replay of a whole tower for small batches (launch-bound regime; config 1 is B=4): the second call of a
   // (tower, batch, dtype | length) shape is stream-captured from fixed staging buffers, later calls replay it.
@@ -254,18 +248,6 @@ struct jimm_model {
 namespace jimm {
 
 static size_t cdt_size(const jimm_model* m) { return dtype_size(m->cdt); }
-
-// zeroed completion counters for the fused LayerNorm of a residual stream of `rows` rows (null when fusion is off)
-static int alloc_ln_counters(jimm_model* m, size_t rows, int** out) {
-  *out = nullptr;
-  if (!m->fuse_ln || m->simt || m->epi_mode_res != 2) return 0;
-  const size_t n = (rows + 31) / 32 + 1;
-  void* p = nullptr;
-  if (int rc = m->pool.alloc(&p, n * sizeof(int))) return rc;
-  JIMM_CUDA_CHECK(cudaMemset(p, 0, n * sizeof(int)));
-  *out = static_cast<int*>(p);
-  return 0;
-}
 
 // ------------------------------------------------------------------------------------------
 // parameter upload / packing helpers (finalize)
@@ -492,32 +474,22 @@ struct EncBufs {  // the activation buffers one encoder stack works in
   float* x;
   void* h;
   void* big;
-  int* ln_cnt;  // completion counters of the fused LayerNorm (one per 32 rows; null = LayerNorm stays a kernel)
 };
 
 static int plan_encoder(jimm_model* m, Encoder* enc, int Tmax, EncBufs ws) {
   const EncoderCfg& c = enc->c;
   const int act = c.act == JIMM_QUICK_GELU ? ACT_QUICK_GELU : ACT_GELU_TANH;
-  // x + attn(norm1(x)) is followed by norm2, x + mlp(norm2(x)) by the NEXT block's norm1 (common/transformer.py:130-131): the residual
-  // GEMMs normalise the rows they complete and write the next GEMM's A operand, so only the first norm1 of a stack is a kernel
-  auto with_ln = [&](GemmEpilogue e, const LNW& ln) {
-    if (ws.ln_cnt) { e.ln_scale = ln.scale; e.ln_bias = ln.bias; e.ln_out = ws.h; e.ln_out_type = m->cdt; e.ln_ldo = c.D; e.ln_eps = c.eps; e.ln_cnt = ws.ln_cnt; }
-    return e;
-  };
-  for (size_t bi = 0; bi < enc->blocks.size(); ++bi) {
-    BlockW& b = enc->blocks[bi];
+  for (BlockW& b : enc->blocks) {
     // QKV: h[T,D] x Wqkv[3D,D]^T + b -> qkv (16-bit) [T,3D]
     JIMM_TRY(gemm_plan_init(&b.p_qkv, m->cdt, ws.h, c.D, b.qkv.w, c.D, Tmax, 3 * c.D, c.D,
                             epi_plain(b.qkv, ACT_NONE, ws.big, m->adt, 3 * c.D, m->epi_mode_16)));
     // out-proj: attn[T,D] x Wo[D,D]^T + bo + x -> x
-    JIMM_TRY(gemm_plan_init(&b.p_out, m->cdt, ws.h, c.D, b.out.w, c.D, Tmax, c.D, c.D, with_ln(epi_residual(b.out, ws.x, c.D, m->epi_mode_res), b.norm2)));
+    JIMM_TRY(gemm_plan_init(&b.p_out, m->cdt, ws.h, c.D, b.out.w, c.D, Tmax, c.D, c.D, epi_residual(b.out, ws.x, c.D, m->epi_mode_res)));
     // FC1: h x W1^T + b1 -> act -> mid [T,M]
     JIMM_TRY(gemm_plan_init(&b.p_fc1, m->cdt, ws.h, c.D, b.fc1.w, c.D, Tmax, c.M, c.D,
                             epi_plain(b.fc1, act, ws.big, m->cdt, c.M, m->epi_mode_16)));
     // FC2: mid x W2^T + b2 + x -> x
-    GemmEpilogue e2 = epi_residual(b.fc2, ws.x, c.D, m->epi_mode_res);
-    if (bi + 1 < enc->blocks.size()) e2 = with_ln(e2, enc->blocks[bi + 1].norm1);
-    JIMM_TRY(gemm_plan_init(&b.p_fc2, m->cdt, ws.big, c.M, b.fc2.w, c.M, Tmax, c.D, c.M, e2));
+    JIMM_TRY(gemm_plan_init(&b.p_fc2, m->cdt, ws.big, c.M, b.fc2.w, c.M, Tmax, c.D, c.M, epi_residual(b.fc2, ws.x, c.D, m->epi_mode_res)));
   }
   return 0;
 }
@@ -543,17 +515,14 @@ static int run_encoder(jimm_model* m, Encoder* enc, int B, int S, cudaStream_t s
   // starts on the data written last -- the part of the 77-310 MB activation still resident in the 126 MB L2.
   int dir = m->l2_alternate ? 1 : 0;  // the patch GEMM / embedding kernels ran forward -> the first LayerNorm runs backward
   auto flip = [&]() { const int d = dir; if (m->l2_alternate) dir ^= 1; return d; };
-  bool h_ready = false;  // ws.h already holds norm1(x) of the coming block (written by the previous block's FC2 epilogue)
   for (BlockW& b : enc->blocks) {
-    if (!h_ready) JIMM_TRY(layernorm_run(ws.x, c.D, 1, 0, nullptr, b.norm1.scale, b.norm1.bias, c.eps, ws.h, m->cdt, c.D, T, c.D, s, flip()));
+    JIMM_TRY(layernorm_run(ws.x, c.D, 1, 0, nullptr, b.norm1.scale, b.norm1.bias, c.eps, ws.h, m->cdt, c.D, T, c.D, s, flip()));
     JIMM_TRY(run_gemm(m, b.p_qkv, ws.h, c.D, b.qkv, T, s, flip()));
     JIMM_TRY(attention_run(ws.big, m->adt, ws.h, m->cdt, B, S, c.H, c.causal, s, flip()));
-    JIMM_TRY(run_gemm(m, b.p_out, ws.h, c.D, b.out, T, s, flip()));  // + residual (+ norm2 -> ws.h when fused)
-    if (m->simt || !gemm_fuses_ln(&b.p_out, T))
-      JIMM_TRY(layernorm_run(ws.x, c.D, 1, 0, nullptr, b.norm2.scale, b.norm2.bias, c.eps, ws.h, m->cdt, c.D, T, c.D, s, flip()));
+    JIMM_TRY(run_gemm(m, b.p_out, ws.h, c.D, b.out, T, s, flip()));  // + residual
+    JIMM_TRY(layernorm_run(ws.x, c.D, 1, 0, nullptr, b.norm2.scale, b.norm2.bias, c.eps, ws.h, m->cdt, c.D, T, c.D, s, flip()));
     JIMM_TRY(run_gemm(m, b.p_fc1, ws.h, c.D, b.fc1, T, s, flip()));
-    JIMM_TRY(run_gemm(m, b.p_fc2, ws.big, c.M, b.fc2, T, s, flip()));  // + residual (+ the next block's norm1 -> ws.h when fused)
-    h_ready = !m->simt && gemm_fuses_ln(&b.p_fc2, T);
+    JIMM_TRY(run_gemm(m, b.p_fc2, ws.big, c.M, b.fc2, T, s, flip()));  // + residual
   }
   return 0;
 }
@@ -589,7 +558,7 @@ static int run_vision(jimm_model* m, const void* img, int in_dtype, int B, float
     if (v.pooling == JIMM_POOL_CLS) JIMM_TRY(cls_row_run(ws.x, v.cls, v.pos, B, S, D, s));
   }
   if (v.pre_norm) JIMM_TRY(layernorm_run(ws.x, D, 1, 0, nullptr, v.ln_pre.scale, v.ln_pre.bias, v.eps_outer, ws.x, DT_F32, D, B * S, D, s));
-  JIMM_TRY(run_encoder(m, &v.enc, B, S, s, EncBufs{ws.x, ws.h, ws.big, ws.ln_cnt}));
+  JIMM_TRY(run_encoder(m, &v.enc, B, S, s, EncBufs{ws.x, ws.h, ws.big}));
   if (v.pooling == JIMM_POOL_CLS) {
     // ln_post is per-row, only row 0 of each sample is consumed (common/vit.py:244-246)
     if (v.head.N > 0) {
@@ -613,7 +582,7 @@ static int run_text(jimm_model* m, const int32_t* ids, int B, int T, float* out,
   TextTower& t = m->txt;
   TextWs& ws = m->wt;
   JIMM_TRY(embed_run(ids, t.table, t.pos, ws.x, B, T, t.D, t.V, s));
-  JIMM_TRY(run_encoder(m, &t.enc, B, T, s, EncBufs{ws.x, ws.h, ws.big, ws.ln_cnt}));
+  JIMM_TRY(run_encoder(m, &t.enc, B, T, s, EncBufs{ws.x, ws.h, ws.big}));
   if (t.pool == JIMM_TPOOL_EOT_ARGMAX) {
     JIMM_TRY(argmax_ids_run(ids, ws.idx, B, T, s));
     JIMM_TRY(layernorm_run(ws.x, t.D, T, 0, ws.idx, t.ln_final.scale, t.ln_final.bias, t.eps_outer, ws.pooled, m->cdt, t.D, B, t.D, s));
@@ -758,8 +727,7 @@ static int finalize_sub(jimm_model* m, int max_batch) {
   JIMM_TRY(m->pool.alloc(&ws.mid2, Bm * 4 * D * cs));
   ws.out_dev_elems = Bm * D;
   JIMM_TRY(m->pool.alloc(&p, ws.out_dev_elems * sizeof(float))); ws.out_dev = static_cast<float*>(p);
-  JIMM_TRY(alloc_ln_counters(m, Tv, &ws.ln_cnt));
-  if (c.kind == JIMM_ENCODER) JIMM_TRY(plan_encoder(m, &v.enc, static_cast<int>(Tv), EncBufs{ws.x, ws.h, ws.big, ws.ln_cnt}));
+  if (c.kind == JIMM_ENCODER) JIMM_TRY(plan_encoder(m, &v.enc, static_cast<int>(Tv), EncBufs{ws.x, ws.h, ws.big}));
   else JIMM_TRY(plan_map_head(m, static_cast<int>(Bm), static_cast<int>(Tv)));
   JIMM_CUDA_CHECK(cudaDeviceSynchronize());
   m->graph_max_batch = 0;
@@ -776,7 +744,7 @@ static int finalize_sub(jimm_model* m, int max_batch) {
 extern "C" {
 
 const char* jimm_last_error(void) { return g_err; }
-int jimm_abi_version(void) { return 1; }
+int jimm_abi_version(void) { return 2; }
 long long jimm_launch_count(void) { return g_launches.load(); }
 long long jimm_graph_replay_count(void) { return g_graph_replays.load(); }
 
@@ -836,7 +804,6 @@ int jimm_model_create(const jimm_config_t* cfg, int device, jimm_model_t** out) 
   if ((env = getenv("JIMM_L2_ALTERNATE"))) m->l2_alternate = atoi(env) != 0;
   if ((env = getenv("JIMM_GRAPH_MAX_BATCH"))) m->graph_max_batch = atoi(env) > 0 ? atoi(env) : 0;
   if ((env = getenv("JIMM_DUAL_STREAMS"))) m->dual_streams = atoi(env) != 0;
-  if ((env = getenv("JIMM_FUSE_LN"))) m->fuse_ln = atoi(env) != 0;
   if ((env = getenv("JIMM_EPI_MODE_16"))) m->epi_mode_16 = atoi(env);
   if ((env = getenv("JIMM_EPI_MODE_RES"))) m->epi_mode_res = atoi(env);
   *out = m;
@@ -1010,15 +977,13 @@ int jimm_model_finalize(jimm_model_t* m, int max_batch) {
     e.rows_in = v.n; e.rows_out = v.S; e.row_off = v.pooling == JIMM_POOL_CLS ? 1 : 0; e.mode = 0;
     JIMM_TRY(gemm_plan_init(&v.p_patch, m->cdt, ws.big, PPC, v.patch.w, PPC, static_cast<int>(Bm) * v.n, D, PPC, e));
   }
-  JIMM_TRY(alloc_ln_counters(m, Tv, &ws.ln_cnt));
-  JIMM_TRY(plan_encoder(m, &v.enc, static_cast<int>(Tv), EncBufs{ws.x, ws.h, ws.big, ws.ln_cnt}));
+  JIMM_TRY(plan_encoder(m, &v.enc, static_cast<int>(Tv), EncBufs{ws.x, ws.h, ws.big}));
   if (v.head.N > 0)
     JIMM_TRY(gemm_plan_init(&v.p_head, m->cdt, ws.pooled, D, v.head.w, D, static_cast<int>(Bm), v.head.N, D,
                             epi_plain(v.head, ACT_NONE, ws.out_dev, DT_F32, v.head.N, 0)));
   if (v.pooling == JIMM_POOL_MAP) JIMM_TRY(plan_map_head(m, static_cast<int>(Bm), static_cast<int>(Tv)));
   if (dual) {
-    JIMM_TRY(alloc_ln_counters(m, Bm * t.T, &m->wt.ln_cnt));
-    JIMM_TRY(plan_encoder(m, &t.enc, static_cast<int>(Bm) * t.T, EncBufs{m->wt.x, m->wt.h, m->wt.big, m->wt.ln_cnt}));
+    JIMM_TRY(plan_encoder(m, &t.enc, static_cast<int>(Bm) * t.T, EncBufs{m->wt.x, m->wt.h, m->wt.big}));
     JIMM_TRY(gemm_plan_init(&t.p_head, m->cdt, m->wt.pooled, t.D, t.head.w, t.D, static_cast<int>(Bm), t.D, t.D,
                             epi_plain(t.head, ACT_NONE, ws.out_dev, DT_F32, t.D, 0)));
   }
@@ -1174,7 +1139,7 @@ int jimm_encoder_forward(jimm_model_t* m, const float* x, int B, int S, float* o
   for (int b0 = 0; b0 < B; b0 += m->max_batch) {
     const int nb = B - b0 < m->max_batch ? B - b0 : m->max_batch;
     JIMM_CUDA_CHECK(cudaMemcpyAsync(m->ws.x, x + b0 * row, nb * row * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    JIMM_TRY(run_encoder(m, &m->vis.enc, nb, S, s, EncBufs{m->ws.x, m->ws.h, m->ws.big, m->ws.ln_cnt}));
+    JIMM_TRY(run_encoder(m, &m->vis.enc, nb, S, s, EncBufs{m->ws.x, m->ws.h, m->ws.big}));
     JIMM_CUDA_CHECK(cudaMemcpyAsync(out + b0 * row, m->ws.x, nb * row * sizeof(float), cudaMemcpyDeviceToDevice, s));
   }
   return 0;
@@ -1483,18 +1448,6 @@ int jimm_k_gemm_ex(int dtype, const void* A, int lda, const void* B, int ldb, in
   JIMM_TRY(gemm_plan_init(&p, dtype, A, lda, B, ldb, M, N, K, e));
   if (tok_pad > 0 && p.epi.mode != 2) { set_last_error("jimm_k_gemm_ex: token-scatter epilogue unavailable (alignment)"); return JIMM_EINVAL; }
   return gemm_plan_run(&p, run_M > 0 ? run_M : M, static_cast<cudaStream_t>(stream), reverse != 0);
-}
-int jimm_k_gemm_residual_ln(int dtype, const void* A, int lda, const void* B, int ldb, int M, int N, int K, const float* bias, float* x, int ldx,
-                            const float* ln_scale, const float* ln_bias, float eps, void* ln_out, int ln_out_type, int ln_ldo, int* counters,
-                            void* stream) {
-  GemmEpilogue e;
-  e.bias = bias; e.residual = x; e.ldr = ldx; e.out = x; e.out_type = DT_F32; e.ldo = ldx; e.mode = 2;
-  e.ln_scale = ln_scale; e.ln_bias = ln_bias; e.ln_out = ln_out; e.ln_out_type = ln_out_type == JIMM_F32 ? DT_TF32 : ln_out_type; e.ln_ldo = ln_ldo;
-  e.ln_eps = eps; e.ln_cnt = counters;
-  GemmPlan p;
-  JIMM_TRY(gemm_plan_init(&p, dtype, A, lda, B, ldb, M, N, K, e));
-  if (!gemm_fuses_ln(&p, M)) { set_last_error("jimm_k_gemm_residual_ln: this shape does not take the fused path (needs M >= 512, N %% 4 == 0, aligned operands)"); return JIMM_EINVAL; }
-  return gemm_plan_run(&p, M, static_cast<cudaStream_t>(stream));
 }
 int jimm_k_layernorm(const float* x, int ldx, int group, int row_off, const int32_t* row_index, const float* scale, const float* bias,
                      float eps, void* out, int out_type, int ldy, int rows, int D, void* stream) {

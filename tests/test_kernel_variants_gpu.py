@@ -354,16 +354,14 @@ def _attn_ref(qkv, B, S, H, causal):
 
 def _attn_cases():
     for S, causal in ((1, 0), (77, 1), (197, 0), (256, 0), (577, 0), (1024, 0)):
-        for impl in ("default", "split", "flash"):
-            if impl == "split" and S > 256:
-                continue  # the split variant is an S <= 256 kernel; above it runs the default kernels
+        for impl in ("default", "flash"):
             yield S, causal, impl
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("S,causal,impl", list(_attn_cases()))
 def test_attention_reverse_and_tf32(lib, monkeypatch, S, causal, impl):
-    """Every attention kernel (tcgen05 S <= 256, its split variant, the long-sequence kernel, the mma.sync flash kernel) with more
+    """Every attention kernel (tcgen05 S <= 256, the long-sequence kernel, the mma.sync flash kernel) with more
     (sample, head) items than SMs: reverse = 1 gives the bits of reverse = 0; fp16 in / tf32 out stores tf32 values within one tf32 ulp
     of the same kernel's fp32 output, which is within the attention bound of the fp64 reference."""
     if impl != "default":

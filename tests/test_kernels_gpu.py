@@ -180,22 +180,6 @@ def test_attention_flash_kernel_forced(lib, monkeypatch, S, causal):
     assert rel_err(out, _attn_ref(qkv, B, S, H, causal)) < 3e-3
 
 
-@pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16])
-@pytest.mark.parametrize("S,causal", [(1, 0), (16, 1), (33, 0), (50, 0), (64, 1), (77, 1), (128, 0), (129, 1), (160, 0), (192, 1), (197, 0), (224, 0), (225, 1), (256, 0), (256, 1)])
-def test_attention_split_variant(lib, monkeypatch, dtype, S, causal):
-    """JIMM_ATTN_IMPL=split: the two-threads-per-row variant of the S <= 256 tcgen05 kernel (slower, kept for A/B runs;
-    profiles/r2_b_attention.md) -- every chunk split nA/nB = 1/0 .. 4/4, both output widths, more items than SMs."""
-    monkeypatch.setenv("JIMM_ATTN_IMPL", "split")
-    B, H = 30, 6
-    qkv = (torch.randn(B * S, 3 * H * 64, device=DEV) * 1.5).to(dtype)
-    ref = _attn_ref(qkv, B, S, H, causal)
-    tol = 3e-3 if dtype == torch.float16 else 2e-2
-    for out_dtype in (dtype, torch.float32):
-        out = torch.empty(B * S, H * 64, dtype=out_dtype, device=DEV)
-        check(lib, lib.jimm_k_attention(ptr(qkv), CODE[dtype], ptr(out), CODE[out_dtype], B, S, H, causal, stream()))
-        assert rel_err(out, ref) < tol, (S, causal, out_dtype, rel_err(out, ref))
-
-
 def test_attention_many_items_persistent(lib):
     """More (sample, head) items than SMs: exercises the persistent loop, the 2-deep smem ring and TMEM slot reuse."""
     B, S, H = 40, 197, 12
@@ -327,42 +311,3 @@ def test_bad_arguments_return_errors(lib):
     rc = lib.jimm_k_layernorm(ptr(x), 6, 1, 0, None, ptr(x), ptr(x), 1e-6, ptr(x), F32, 6, 2, 6, stream())
     assert rc == -1
 
-
-@pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16, torch.float32])
-@pytest.mark.parametrize("M,N,K", [(1000, 768, 256), (50432 // 8, 768, 768), (2000, 512, 2048), (777, 1152, 320), (5000, 1024, 512),
-                                   (1024, 128, 256), (1536, 256, 256), (1000, 384, 512), (2048, 1280, 320), (1024, 1536, 256), (600, 2048, 256)])
-def test_gemm_residual_with_fused_layernorm(lib, dtype, M, N, K):
-    """x += A B^T + bias, then LayerNorm(x) written by the warp that completes each 32-row group (also in place over the A operand, as the
-    out-projection does): x bit-identical to the unfused kernel, the normalised rows equal to the LayerNorm kernel on that x."""
-    torch.manual_seed(M + N)
-    A = torch.randn(M, K, device=DEV).to(dtype)
-    if dtype == torch.float32:
-        A = (A.view(torch.int32) & ~0x1FFF).view(torch.float32)
-    Bw = (torch.randn(N, K, device=DEV) / K ** 0.5).to(dtype)
-    bias = torch.randn(N, device=DEV)
-    x0 = torch.randn(M, N, device=DEV) * 2 + 0.5
-    scale, lbias = torch.randn(N, device=DEV), torch.randn(N, device=DEV)
-    x_ref = gemm(lib, A, Bw, bias=bias, residual=x0.clone(), mode=2)
-    h_ref = torch.empty(M, N, dtype=dtype, device=DEV)
-    oc = CODE[dtype]
-    check(lib, lib.jimm_k_layernorm(ptr(x_ref), N, 1, 0, None, ptr(scale), ptr(lbias), 1e-6, ptr(h_ref), oc, N, M, N, stream()))
-    cnt = torch.zeros(M // 32 + 2, dtype=torch.int32, device=DEV)
-    for rep in range(2):  # second launch: the kernel left its counters at zero
-        x = x0.clone()
-        h = torch.full((M, N), 7.0, dtype=dtype, device=DEV)
-        check(lib, lib.jimm_k_gemm_residual_ln(CODE[A.dtype], ptr(A), K, ptr(Bw), K, M, N, K, ptr(bias), ptr(x), N, ptr(scale), ptr(lbias), 1e-6,
-                                               ptr(h), oc, N, ptr(cnt), stream()))
-        torch.cuda.synchronize()
-        assert torch.equal(x, x_ref), f"rep {rep}: residual stream differs from the unfused kernel"
-        # same arithmetic as layernorm_kernel (the fp32 mode stores tf32-rounded values): equal up to one rounding of the output type
-        tol = {torch.float32: 1e-3, torch.float16: 1e-3, torch.bfloat16: 8e-3}[dtype]
-        assert rel_err(h, h_ref) < tol, f"rep {rep}: fused LayerNorm differs from the LayerNorm kernel: {rel_err(h, h_ref):.2e}"
-        assert float((h.float() != h_ref.float()).float().mean()) < 0.01 or dtype == torch.float32
-        assert int(cnt.abs().sum()) == 0
-    if K == N and dtype != torch.float32:  # in place over the A operand (out-projection: ws.h is both A and the LayerNorm output)
-        x = x0.clone()
-        Ah = A.clone()
-        check(lib, lib.jimm_k_gemm_residual_ln(CODE[A.dtype], ptr(Ah), K, ptr(Bw), K, M, N, K, ptr(bias), ptr(x), N, ptr(scale), ptr(lbias), 1e-6,
-                                               ptr(Ah), oc, N, ptr(cnt), stream()))
-        torch.cuda.synchronize()
-        assert torch.equal(x, x_ref) and rel_err(Ah, h_ref) < tol

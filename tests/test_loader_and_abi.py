@@ -16,7 +16,8 @@ import jimm_oracle as O
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_abi_exports_every_declared_symbol(lib):
+def test_abi_v2_exports_every_declared_symbol(lib):
+    """ABI version 2: the header, the ctypes bindings and the library's exports name the same entry points."""
     from jimm_b200 import _lib
 
     header = open(os.path.join(ROOT, "include", "jimm_b200.h")).read()
@@ -26,7 +27,7 @@ def test_abi_exports_every_declared_symbol(lib):
     assert declared == set(_lib.SIGNATURES), (declared ^ set(_lib.SIGNATURES))
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.jimm_abi_version() == 1
+    assert lib.jimm_abi_version() == 2
     assert lib.jimm_launch_count() >= 0
 
 

@@ -110,21 +110,6 @@ def test_vit_b16_batch4(vitb16, dtype):
     assert torch.equal(out_n, out.cpu())
 
 
-@pytest.mark.parametrize("dtype", [torch.float16, torch.float32])
-def test_vit_b16_fused_layernorm_opt_in(vitb16, dtype, monkeypatch):
-    """JIMM_FUSE_LN=1 (the out-proj / FC2 GEMMs normalise the rows they complete; off by default because it is slower, DESIGN.md section 3)
-    is the same function: within the parity bound of the oracle and within rounding noise of the default path."""
-    from jimm_b200.models import VisionTransformer
-
-    cfg, p, img, ref = vitb16
-    base = _set(VisionTransformer(dtype=dtype), p).eval()(img.cuda())
-    monkeypatch.setenv("JIMM_FUSE_LN", "1")  # read when the native model is created
-    out = _set(VisionTransformer(dtype=dtype), p).eval()(img.cuda())
-    check_parity("c1 ViT-B/16@224 B=4, JIMM_FUSE_LN=1", "logits", dtype, "fp32", out, ref, TOL)
-    assert (out - base).abs().max().item() < 2e-4
-    assert torch.equal(out.argmax(-1), base.argmax(-1))
-
-
 def test_vit_b16_batch256_fp16_config2():
     """BASELINE config 2 at full size: ViT-B/16 @224, batch 256, fp16 operands -- logits within 1e-3 of the fp32 oracle,
     identical argmax (the oracle forward of 256 images takes ~10-60 s of host time)."""
